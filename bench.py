@@ -2,14 +2,16 @@
 """
 bench.py — 16384-sample frames/s of the Wave-U-Net forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision fp32|bf16|auto]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision fp32|bf16|auto] [--dump-outputs DIR]
     python bench.py --impl reference ...        # the reference's CPU implementation of the path (host cores)
     python bench.py --mode train   [--batch 64] # SURVEY §8f N1 / configs[4]: fwd + bwd + Adam per step, grads all-reduced
     python bench.py --mode enhance              # configs[3]: 10 s clips through enhance_waveforms, 1024 frames/step sharded
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W   # one rank per GPU, batch sharded, no collective on the path
 
-A "step" is one forward over one batch of B synthetic frames per GPU ([B,1,16384] fp32, eval mode).
+A "step" is one forward over one batch of B synthetic frames per GPU ([B,1,16384] fp32, eval mode). --steps is the number
+of timed steps in every mode. --dump-outputs DIR writes what the last timed forward returned on rank 0 to DIR/output.npy
+(float32); the weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 Workload at N=1 = BASELINE.json configs[2] shape (batch 256, 16384 samples, 12 levels); weak scaling:
 every rank runs the same B.  One JSON line is printed by rank 0.
 """
@@ -131,15 +133,14 @@ class ClockSampler:
 # ------------------------------------------------------------------------------------------------
 # CPU baseline: the reference forward restated with torch ops (oracle/wunet_oracle.torch_port_forward)
 # ------------------------------------------------------------------------------------------------
-def cpu_reference_run(iters: int, warmup: int, budget_s: float):
+def cpu_reference_run(iters: int, warmup: int):
     """BASELINE.json configs[0] (batch 1) and a batch of 8 frames, fp32, on the host cores: the thread count is chosen by a
-    short sweep and set explicitly (under torch.distributed.run the environment carries OMP_NUM_THREADS=1), then >= 20 timed
+    short sweep and set explicitly (under torch.distributed.run the environment carries OMP_NUM_THREADS=1), then `iters` timed
     forwards per batch size; best and median are reported, `value` = the better of the two batch sizes by its MEDIAN."""
     from oracle import wunet_oracle as wo
     st = {k: torch.from_numpy(np.asarray(v)) for k, v in wo.make_state(N_LAYERS, CH_INT, seed=0).items()}
     ncpu = os.cpu_count() or 1
     cands = sorted({t for t in (8, 16, 32, 64) if t <= ncpu} | {min(ncpu, 8)})
-    t_start = time.perf_counter()
     out = {}
     with torch.no_grad():
         for fps in (1, 8):
@@ -160,7 +161,7 @@ def cpu_reference_run(iters: int, warmup: int, budget_s: float):
             for _ in range(max(3, warmup)):
                 wo.torch_port_forward(st, x)
             ts = []
-            while len(ts) < max(20, iters) and (len(ts) < 20 or time.perf_counter() - t_start < budget_s):
+            for _ in range(iters):
                 t0 = time.perf_counter()
                 wo.torch_port_forward(st, x)
                 ts.append(time.perf_counter() - t0)
@@ -223,6 +224,22 @@ def incumbent_run(st, B, dev, iters=5, warm=3):
     return res
 
 
+DUMP_LIMIT = 64 * 10**6                                      # bytes written by --dump-outputs
+
+
+def dump_output(out_dir: str, y: torch.Tensor) -> None:
+    """y ([B,1,T], what model(x) returned) as out_dir/output.npy in float32. Above DUMP_LIMIT a fixed, seeded sample of the
+    frames is written instead, and their indices (ascending) as out_dir/output_frames.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    a = y.detach().float().cpu().numpy()
+    keep = DUMP_LIMIT // (a[0].nbytes + 8)
+    if keep < len(a):
+        frames = np.sort(np.random.default_rng(0).choice(len(a), size=keep, replace=False))
+        np.save(os.path.join(out_dir, "output_frames.npy"), frames.astype(np.float64))
+        a = a[frames]
+    np.save(os.path.join(out_dir, "output.npy"), a)
+
+
 def time_steps(fn, steps, warm=3):
     """ms per call of fn() over `steps` back-to-back calls (CUDA events on the current stream)"""
     for _ in range(warm):
@@ -270,7 +287,7 @@ def run_train(ctx):
     from wave_u_net_for_speech_enhancement_b200 import Model, _lib
     from wave_u_net_for_speech_enhancement_b200.train_step import GradientBucket
     B = args.batch or 64
-    steps = min(args.steps, 20)
+    steps = args.steps
     model = Model(N_LAYERS, CH_INT)
     model.load_state_dict(st, strict=True)
     model = model.to(dev).train()
@@ -404,7 +421,7 @@ def run_enhance(ctx):
     args, rank, world, dev, dist, emit, st = (ctx[k] for k in ("args", "rank", "world", "dev", "dist", "emit", "st"))
     from wave_u_net_for_speech_enhancement_b200 import Model, _lib, enhance
     per_gpu = args.batch or 128
-    steps = min(args.steps, 20)
+    steps = args.steps
     clips_per_step = max(1, (per_gpu * world) // 10)
     rng = np.random.default_rng(7)
     clips = [(0.3 * rng.standard_normal(160000)).astype(np.float32) for _ in range(min(clips_per_step, 16))]
@@ -463,7 +480,12 @@ def main():
     ap.add_argument("--precision", default="auto", choices=["auto", "fp32", "bf16"])
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed forward to DIR/output.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "forward" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the forward of the b200 implementation (--mode forward --impl b200)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -484,7 +506,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        r = cpu_reference_run(iters=min(args.steps, 60), warmup=args.warmup, budget_s=100.0)
+        r = cpu_reference_run(iters=args.steps, warmup=args.warmup)
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "frames/s", "n_gpus": args.gpus,
                 "steps": r["steps_done"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -564,7 +586,7 @@ def main():
         sampler.start()
     e0.record()
     for i in range(args.steps):
-        step(i)
+        y = step(i)
     e1.record()
     torch.cuda.synchronize()
     ms_total = e0.elapsed_time(e1)
@@ -713,7 +735,7 @@ def main():
             extras["incumbent"]["speedup_vs_best_mode"] = round(value / max(extras["incumbent"][k]["frames_per_s"]
                                                                              for k in ("fp32", "tf32", "bf16_autocast")), 1)
         if not args.no_cpu_baseline:
-            r = cpu_reference_run(iters=20, warmup=2, budget_s=25.0)
+            r = cpu_reference_run(iters=20, warmup=2)
             cpu = {k: r[k] for k in ("value", "unit", "cores", "kind", "sample", "batch1", "batch8")}
 
     line = {
@@ -740,6 +762,8 @@ def main():
         line["cpu_baseline"] = cpu
     line.update(extras)
     line["library"] = _lib.load().wunet_version().decode()
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     emit(line)
     if dist is not None:
         dist.destroy_process_group()

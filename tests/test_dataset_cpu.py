@@ -1,10 +1,10 @@
 """Training-side data path (SURVEY §8f row N4): the native wav reader + aligned random crop against the reference's
 `dataset/waveform_dataset.py:56-67` / `util/utils.py:101-113`. CPU only. The wav files are written here with scipy / the
-stdlib; where `/root/reference` exists the UNCHANGED reference Dataset class is driven next to the drop-in (its `librosa.load`
-stubbed with a scipy reader that converts like soundfile does), with the same numpy seed."""
+stdlib. What the UNCHANGED reference Dataset class returned for them (its `librosa.load` stubbed with a scipy reader that
+converts like soundfile does), with the same numpy seed, is stored in tests/golden/dataset_items.json."""
+import hashlib
+import json
 import os
-import sys
-import types
 import wave
 
 import torch
@@ -15,8 +15,6 @@ import scipy.io.wavfile as wavfile
 
 from wave_u_net_for_speech_enhancement_b200 import _lib
 from wave_u_net_for_speech_enhancement_b200 import dataset as ds
-
-REF = "/root/reference"
 
 
 def soundfile_like(path):
@@ -131,35 +129,19 @@ def test_dataset_items_and_crops(tmp_path):
         ds.Dataset(lst, sample_length=30000)[0]                   # clip shorter than sample_length: the reference asserts too
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "dataset")), reason="reference checkout not present on this box")
-def test_dataset_matches_unchanged_reference_class(tmp_path, monkeypatch):
+def test_dataset_matches_unchanged_reference_class(tmp_path, golden_dir):
     lst, _lines = _pair_files(tmp_path)
-    stub = types.ModuleType("librosa")
-    stub.load = lambda path, sr=None: soundfile_like(path)
-    monkeypatch.setitem(sys.modules, "librosa", stub)
-    for name in ("pesq", "pystoi", "pystoi.stoi"):
-        m = types.ModuleType(name)
-        m.pesq = m.stoi = lambda *a, **k: 0.0
-        monkeypatch.setitem(sys.modules, name, m)
-    sys.modules["pystoi"].stoi = sys.modules["pystoi.stoi"]
-    monkeypatch.syspath_prepend(REF)
-    for name in [k for k in sys.modules if k.split(".")[0] in ("util", "dataset")]:
-        monkeypatch.delitem(sys.modules, name)
-    import importlib
-    ref_ds = importlib.import_module("dataset.waveform_dataset")
-    try:
-        for mode in ("train", "validation"):
-            r = ref_ds.Dataset(lst, sample_length=16384, mode=mode)
-            o = ds.Dataset(lst, sample_length=16384, mode=mode)
-            np.random.seed(7)
-            want = [r[i] for i in range(len(r))]
-            np.random.seed(7)
-            got = [o[i] for i in range(len(o))]
-            for (wm, wc, wn), (gm, gc, gn) in zip(want, got):
-                assert wn == gn and wm.shape == gm.shape and np.array_equal(wm, gm) and np.array_equal(wc, gc)
-    finally:
-        for name in [k for k in sys.modules if k.split(".")[0] in ("util", "dataset")]:
-            sys.modules.pop(name, None)
+    want = json.load(open(os.path.join(golden_dir, "dataset_items.json")))
+    for mode in ("train", "validation"):
+        o = ds.Dataset(lst, sample_length=want["sample_length"], mode=mode)
+        np.random.seed(want["seed"])
+        got = [o[i] for i in range(len(o))]
+        assert len(got) == len(want[mode])
+        for w, (gm, gc, gn) in zip(want[mode], got):
+            assert gn == w["name"] and list(gm.shape) == w["shape"] and list(gc.shape) == w["shape"]
+            assert str(gm.dtype) == str(gc.dtype) == w["dtype"]
+            assert hashlib.sha256(np.ascontiguousarray(gm).tobytes()).hexdigest() == w["mixture_sha256"], (mode, gn)
+            assert hashlib.sha256(np.ascontiguousarray(gc).tobytes()).hexdigest() == w["clean_sha256"], (mode, gn)
 
 
 @pytest.mark.parametrize("pcm", [False, True])
